@@ -8,7 +8,8 @@ synthetic text_embeds (bs,256,768), random-init weights (final_conv re-randomise
 
     python bench.py --gpus 1 --steps 3 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
-    python bench.py --impl reference ...      # the reference algorithm (oracle port) on this box's host cores
+    python bench.py --impl reference ...      # the reference algorithm (oracle port) on the host cores
+    python bench.py --dump-outputs DIR ...    # also write the last timed step's images as DIR/images.npy (float32)
 
 Prints ONE JSON line (rank 0).  Timing: CUDA events on the launching stream, barrier + synchronize on both sides,
 max over ranks.  `value` = inputs resident in HBM; `e2e` = same call with pinned-host text_embeds copied in and the
@@ -256,6 +257,22 @@ def run_reference(args):
     }))
 
 
+DUMP_MAX_ELEMENTS = (64 << 20) // 4                          # 64 MB of float32
+
+
+def dump_images(out_dir, images):
+    """Writes what sample() returned as out_dir/images.npy (float32), so that two builds run with the same arguments can be
+    compared output for output. Above 64 MB it keeps a fixed, seeded sample of the flattened elements instead: the same
+    positions, in ascending order, for every build."""
+    import numpy as np
+    a = images.detach().float().cpu()
+    if a.numel() > DUMP_MAX_ELEMENTS:
+        keep = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MAX_ELEMENTS].sort().values
+        a = a.reshape(-1)[keep]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'images.npy'), a.numpy())
+
+
 def workload_config(args, desc=None):
     if desc is not None:
         return {'workload': desc + f', random text_embeds ({args.bs},256,768)', 'global_batch': args.bs * args.gpus,
@@ -282,6 +299,7 @@ def main():
     ap.add_argument('--eager-steps', type=int, default=20, help='denoising steps of the in-process eager-PyTorch-on-GPU baseline (0 = skip)')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--eager-gpu', action='store_true', help='with --impl reference: run the oracle port with torch CUDA ops (informational)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the images of the last timed step to DIR/images.npy (float32)')
     args = ap.parse_args()
     defaults = {1: (16, 128, 1000), 2: (64, 128, None), 3: (8, 128, 100), 4: (64, 192, 1000)}[args.config]
     args.bs = args.bs if args.bs is not None else defaults[0]
@@ -310,6 +328,7 @@ def main():
     out_host = torch.empty(args.bs, 3, out_px, out_px).pin_memory()
 
     own_events = []                                             # (before, after) this rank's own sampling work, all-gather excluded
+    last = {}
 
     def step_resident():
         ea, eb = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -319,6 +338,7 @@ def main():
         own_events.append((ea, eb))
         if world > 1:
             img = all_gather_images(img, [args.bs] * world)
+        last['images'] = img
         return img
 
     def step_e2e():
@@ -355,6 +375,8 @@ def main():
     with ClockSampler(local) as clk:
         ms, ms_ranks = timed(step_resident, args.steps)
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:                         # before the e2e steps sample again
+        dump_images(args.dump_outputs, last['images'])
     own_ms = [sum(a.elapsed_time(b) for a, b in own_events) / args.steps]   # this rank's shard alone: a slow GPU shows up by index
     if world > 1:
         own_all = torch.empty(world, device=device)

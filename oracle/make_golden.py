@@ -376,6 +376,8 @@ def main():
     print(f'[configs[0]: dim32 @64, bs 2, 50 DDPM steps] ref-vs-oracle max|d| = {d:.3e}')
     assert d < 1e-3
     big['cfg0_50steps'] = dict(kwargs=kw0, wseed=15, iseed=106, seed=83, timesteps=50, out=r50)
+    # the 256 x 256 output in a file of its own keeps every fixture under 1 MB
+    torch.save(big.pop('srunet256'), os.path.join(out_dir, 'baseline_srunet256.pt'))
     torch.save(big, os.path.join(out_dir, 'baseline_shapes.pt'))
 
     # ---------------------------------------------------------------- 5g. boundary options: attn_dim_head = 32 (the reference's UnetConfig default,

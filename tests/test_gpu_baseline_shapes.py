@@ -1,6 +1,6 @@
 """GPU (-m gpu): parity at the BASELINE.json shapes (VERDICT r01 "next round" item 1).
 
-Single forwards are compared with outputs of the LIVE reference (tests/golden/baseline_shapes.pt, written by
+Single forwards are compared with outputs of the LIVE reference (tests/golden/baseline_*.pt, written by
 oracle/make_golden.py, which also hard-asserts oracle == reference on the same inputs); inputs and weights are rebuilt
 from seeds.  Trajectories are compared with the oracle run on this box's host cores on the SAME CUDA-drawn noise.
 Tolerances: bf16 activations / fp32 accumulation against an fp32 reference, see DESIGN.md section 4; the measured
@@ -82,7 +82,7 @@ def test_cfg5_unet_dim192_forward_matches_reference():
 
 def test_cfg4_srunet256_forward_256px_matches_reference():
     """BASELINE.json configs[3] second stage: SRUnet256(lowres_cond=True) at 256 x 256, B = 1 (memory_efficient, 64 Ki pixel rows)."""
-    g = load_golden('baseline_shapes.pt')['srunet256']
+    g = load_golden('baseline_srunet256.pt')
     u, _ = load_unet(b2.SRUnet256, contract()['srunet256'], g['wseed'], lowres_cond=True)
     x, te, tm = seeded_inputs(g['iseed'], 1, 256)
     low = torch.randn(1, 3, 256, 256, generator=torch.Generator().manual_seed(g['lseed']))

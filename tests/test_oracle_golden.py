@@ -161,11 +161,12 @@ def test_pred_objectives_v_and_x_start_match_reference_golden():
 
 
 def test_baseline_shape_fixture_is_complete():
-    """tests/golden/baseline_shapes.pt holds the live reference's outputs at the BASELINE.json shapes (the GPU suite replays them);
-    here: the fixture's entries and the key->shape contracts they rebuild their weights from."""
+    """tests/golden/baseline_shapes.pt and baseline_srunet256.pt hold the live reference's outputs at the BASELINE.json shapes (the
+    GPU suite replays them); here: the fixture's entries and the key->shape contracts they rebuild their weights from."""
     from tests.helpers import contract
     g, c = load_golden('baseline_shapes.pt'), contract()
-    assert set(g) == {'dim128', 'dim192', 'srunet256', 'srunet1024_upscale', 'cfg0_50steps'}
+    assert set(g) == {'dim128', 'dim192', 'srunet1024_upscale', 'cfg0_50steps'}
+    g['srunet256'] = load_golden('baseline_srunet256.pt')
     assert g['dim128']['out_cond'].shape == (2, 3, 64, 64) and g['dim192']['out_cond'].shape == (1, 3, 64, 64)
     assert g['srunet256']['out'].shape == (1, 3, 256, 256) and g['srunet1024_upscale']['out'].shape == (2, 3, 128, 128)
     assert g['cfg0_50steps']['out'].shape == (2, 3, 64, 64) and g['cfg0_50steps']['timesteps'] == 50
