@@ -75,6 +75,8 @@ SIGNATURES = {
     'b200_conv_gemm_splitk': [_I, _I, _I, _I, _I],
     'b200_conv_gemm': [C.POINTER(Src), _I, C.POINTER(Seg), _I, _I, _I, _I, _P, _I, C.POINTER(Epilogue), _I, _P, _P],
     'b200_attention': [_P, _P, _L, _L, _I, _I, _P, _P, _L, _L, _I, _I, _I, _I, _F, _P],
+    'b200_linear_xattn_context': [_P, _P, _L, _I, _I, _I, _I, _I, _P, _P],
+    'b200_linear_cross_attention': [_P, _P, _L, _I, _I, _P, _I, _I, _I, _P],
     'b200_rmsnorm_film_silu': [C.POINTER(Src), _I, _F, _P, _P, _I, _I, _P, _I, _L, _P],
     'b200_layernorm': [_P, _I, _P, _P, _F, _P, _I, _P, _I, _L, _I, _P],
     'b200_gca_gate': [_P, _I, _I, _I, _I, _P, _F, _P, _P, _I, _P, _P, _P, _I, _P, _P],

@@ -1349,6 +1349,259 @@ cross_attn_tc_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_cons
   }
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// Linear cross-attention (LinearCrossAttention.forward, imagen_pytorch.py:836-874):
+//   out = softmax_d(q) @ C,   C[d, e] = 8 * sum_j softmax_j(k)[j, d] * v[j, e]      (per sample row and head)
+// Unlike CrossAttention there is no per-pixel score matrix: the keys enter only through the dim_head x dim_head matrix C.
+// linear_xattn_context_kernel builds C once per step (the time-token K/V rows change every step) and stores it bf16 as
+// [B][heads][64 d][64 e], the layout of a V tile, so that the main kernel loads it with the same TMA map / MN-major
+// descriptor as cross_attn_tc_kernel's V.  Head channels >= dim_head (zero-padded heads) get C rows of exact zeros.
+// ------------------------------------------------------------------------------------------------------------------
+constexpr int LX_CTX_THREADS = 256;
+constexpr int LX_CTX_SMEM = 2 * 64 * 64 * 4 + 2 * 64 * 4;   // one 64-token chunk of softmax_j(k) and of v (fp32) + column max / scale
+
+__global__ void __launch_bounds__(LX_CTX_THREADS)
+linear_xattn_context_kernel(const __nv_bfloat16* __restrict__ k, const __nv_bfloat16* __restrict__ v, long long kv_bs, int kv_rs, int n_keys,
+                            int dim_head, __nv_bfloat16* __restrict__ ctx) {
+  pdl_trigger();
+  extern __shared__ float lx_smem[];
+  float* sW = lx_smem;               // [64 tokens][64 d]: exp(k - max_d) * 8 / sum_d
+  float* sV = sW + 64 * 64;          // [64 tokens][64 e]
+  float* sMax = sV + 64 * 64;        // [64]
+  float* sScale = sMax + 64;         // [64]
+  const int h = blockIdx.x, b = blockIdx.y, heads = gridDim.x, tid = threadIdx.x;
+  const __nv_bfloat16* kb = k + (long long)b * kv_bs + h * 64;
+  const __nv_bfloat16* vb = v + (long long)b * kv_bs + h * 64;
+  pdl_wait();
+  // column statistics of k over the tokens (softmax over dim -2), fp32 with a true max: the logits are unbounded
+  if (tid < 64) {
+    float m = -INFINITY;
+    for (int j = 0; j < n_keys; ++j) m = fmaxf(m, __bfloat162float(kb[(long long)j * kv_rs + tid]));
+    float s = 0.f;
+    for (int j = 0; j < n_keys; ++j) s += __expf(__bfloat162float(kb[(long long)j * kv_rs + tid]) - m);
+    sMax[tid] = m;
+    sScale[tid] = tid < dim_head ? 8.f / s : 0.f;   // CrossAttention's scale = 8 on q, folded into C (q @ C is linear)
+  }
+  const int e = tid & 63, d0 = tid >> 6;            // this thread: C[d0 + 4 i][e], i < 16
+  float acc[16];
+#pragma unroll
+  for (int i = 0; i < 16; ++i) acc[i] = 0.f;
+  for (int j0 = 0; j0 < n_keys; j0 += 64) {
+    const int nj = n_keys - j0 < 64 ? n_keys - j0 : 64;
+    __syncthreads();                                 // statistics ready / previous chunk consumed
+    for (int idx = tid; idx < nj * 64; idx += LX_CTX_THREADS) {
+      const int j = idx >> 6, c = idx & 63;
+      const long long off = (long long)(j0 + j) * kv_rs + c;
+      sW[idx] = __expf(__bfloat162float(kb[off]) - sMax[c]) * sScale[c];
+      sV[idx] = __bfloat162float(vb[off]);
+    }
+    __syncthreads();
+    for (int j = 0; j < nj; ++j) {
+      const float vv = sV[j * 64 + e];
+#pragma unroll
+      for (int i = 0; i < 16; ++i) acc[i] = fmaf(sW[j * 64 + d0 + 4 * i], vv, acc[i]);
+    }
+  }
+  __nv_bfloat16* cb = ctx + ((long long)b * heads + h) * 64 * 64;
+#pragma unroll
+  for (int i = 0; i < 16; ++i) cb[(d0 + 4 * i) * 64 + e] = __float2bfloat16_rn(acc[i]);
+}
+
+// Main kernel, persistent like cross_attn_tc_kernel: one CTA per SM walks a contiguous range of work items (sample b, 128-row query
+// tile, head h).  The C tiles of all heads of the current sample stay resident in shared memory (8 x 8 KB, reloaded when b changes),
+// q tiles stream through a TMA ring, and LX_NS tensor-memory slots (O 64 columns + P 32 columns) keep LX_NS items in flight:
+//   4 worker warps per slot: q row from shared memory -> softmax over the first dim_head channels in fp32 (one thread per row) ->
+//   P (bf16, exact zeros in padded channels) -> tensor memory  ->  O = P C (TS-form tcgen05.mma, M128 x N64 x K64)  ->
+//   the same warps: tcgen05.ld O -> bf16 -> one 128-byte row store per thread.
+// The softmax already normalises each row and C carries the 8, so O needs no further scaling.
+constexpr int LX_NS = 4;                               // TMEM slots / items in flight
+constexpr int LX_QS = 6;                               // q ring stages
+constexpr int LX_CTX_BYTES = 64 * 64 * 2;              // one head's C tile: 8 KB
+constexpr int LX_MAX_HEADS = 8;
+constexpr int LX_SMEM = LX_QS * FA_Q_BYTES + LX_MAX_HEADS * LX_CTX_BYTES + 1024 + 512;
+
+struct LxParams {
+  __nv_bfloat16* o;
+  long long q_bs;          // elements between samples in q / o
+  int q_rs;                // row stride of q and o (elements); head h starts at column 64 h
+  int rows, B, heads, dim_head;
+  int tiles_per_sample;    // ceil(rows / 128)
+  int items_per_cta;
+  uint32_t wait_ns;
+};
+
+__global__ void __launch_bounds__(64 + 128 * LX_NS, 1)
+linear_cross_attn_tc_kernel(const __grid_constant__ CUtensorMap mapQ, const __grid_constant__ CUtensorMap mapC, const __grid_constant__ LxParams p) {
+  pdl_trigger();
+  extern __shared__ uint8_t fa_smem_raw[];
+  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(fa_smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
+  uint8_t* sQ = smem;                                        // [LX_QS] q tiles
+  uint8_t* sC = sQ + LX_QS * FA_Q_BYTES;                     // [heads] C tiles of the current sample
+  uint64_t* bars = reinterpret_cast<uint64_t*>(sC + LX_MAX_HEADS * LX_CTX_BYTES);
+  uint64_t* q_full = bars;                       // [LX_QS]
+  uint64_t* q_empty = q_full + LX_QS;            // [LX_QS]
+  uint64_t* c_full = q_empty + LX_QS;            // [1]
+  uint64_t* c_empty = c_full + 1;                // [1]
+  uint64_t* p_full = c_empty + 1;                // [LX_NS]
+  uint64_t* o_full = p_full + LX_NS;             // [LX_NS]
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(o_full + LX_NS);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const long long total_items = (long long)p.B * p.tiles_per_sample * p.heads;
+  const long long item0 = (long long)blockIdx.x * p.items_per_cta;
+  const long long item1 = item0 + p.items_per_cta < total_items ? item0 + p.items_per_cta : total_items;
+  const int n_items = item1 > item0 ? (int)(item1 - item0) : 0;
+  const int per_sample = p.tiles_per_sample * p.heads;
+
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&mapQ);
+    tma_prefetch_desc(&mapC);
+    for (int s = 0; s < LX_QS; ++s) { mbar_init(&q_full[s], 1); mbar_init(&q_empty[s], 4); }   // q_empty: one arrival per worker warp
+    mbar_init(c_full, 1);
+    mbar_init(c_empty, 1);
+    for (int s = 0; s < LX_NS; ++s) {
+      mbar_init(&p_full[s], 4);
+      mbar_init(&o_full[s], 1);
+    }
+    fence_barrier_init();
+  }
+  if (warp == 1) tmem_alloc(tmem_slot, 512u);
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);
+  pdl_wait();
+  // TMEM columns: O of slot s at 64 s, the packed P tiles behind them (256 + 32 s)
+  constexpr uint32_t P_BASE = 64 * LX_NS;
+
+  if (warp == 0) {
+    if (elect_one()) {
+      // ---------------- TMA producer: C of all heads whenever the sample changes, then one q tile per item
+      int cur_b = -1, epoch = 0;
+      for (int i = 0; i < n_items; ++i) {
+        const long long it = item0 + i;
+        const int b = (int)(it / per_sample), rem = (int)(it % per_sample);
+        const int tile = rem / p.heads, h = rem % p.heads;
+        if (b != cur_b) {
+          mbar_wait_sleep(c_empty, (uint32_t)((epoch & 1) ^ 1), p.wait_ns);      // every MMA that read the previous sample's C has completed
+          mbar_expect_tx(c_full, (uint32_t)(p.heads * LX_CTX_BYTES));
+          for (int hh = 0; hh < p.heads; ++hh) tma_load_4d(sC + hh * LX_CTX_BYTES, &mapC, c_full, 0, 0, hh, b);
+          cur_b = b;
+          ++epoch;
+        }
+        const int st = i % LX_QS;
+        mbar_wait_sleep(&q_empty[st], (uint32_t)(((i / LX_QS) & 1) ^ 1), p.wait_ns);
+        mbar_expect_tx(&q_full[st], FA_Q_BYTES);
+        tma_load_4d(sQ + st * FA_Q_BYTES, &mapQ, &q_full[st], 0, h, tile * FA_BM, b);
+      }
+    }
+  } else if (warp == 1) {
+    if (elect_one()) {
+      // ---------------- MMA issuer: O = P C per item, P from tensor memory
+      const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 16) | ((uint32_t)(FA_D >> 3) << 17) | ((uint32_t)(FA_BM >> 4) << 24);
+      int epoch = 0, c_b = -1;
+      for (int i = 0; i < n_items; ++i) {
+        const long long it = item0 + i;
+        const int b = (int)(it / per_sample), h = (int)(it % p.heads);   // per_sample is a multiple of heads
+        const int slot = i % LX_NS;
+        if (b != c_b) {
+          mbar_wait_sleep(c_full, (uint32_t)(epoch & 1), p.wait_ns);
+          c_b = b;
+          ++epoch;
+        }
+        mbar_wait_sleep(&p_full[slot], (uint32_t)((i / LX_NS) & 1), p.wait_ns);
+        tc_fence_after();
+        const uint32_t c_addr = smem_u32(sC + h * LX_CTX_BYTES);
+#pragma unroll
+        for (int k = 0; k < FA_D / 16; ++k) {
+          const uint32_t a_tmem = tmem_base + P_BASE + (uint32_t)(slot * 32 + k * 8);
+          const uint64_t bdesc = make_sw128_mnmajor_desc(c_addr + (uint32_t)(k * 16 * 128), 1024, 1024);
+          umma_bf16_ts(tmem_base + (uint32_t)(slot * 64), a_tmem, bdesc, idesc, k != 0 ? 1u : 0u);
+        }
+        umma_commit(&o_full[slot]);
+        const bool next_same_sample = i + 1 < n_items && (int)((it + 1) / per_sample) == b;
+        if (i + 1 < n_items && !next_same_sample) umma_commit(c_empty);   // this sample's C may be replaced once its MMAs complete
+      }
+    }
+  } else {
+    // ---------------- workers: slot = (warp - 2) / 4, thread = one query row of every item of its slot
+    const int slot = (warp - 2) >> 2;
+    const int q4 = warp & 3;
+    const int r = q4 * 32 + lane;
+    const uint32_t lane_off = (uint32_t)(q4 * 32) << 16;
+    const uint32_t t_o = tmem_base + lane_off + (uint32_t)(slot * 64);
+    const uint32_t t_p = tmem_base + lane_off + P_BASE + (uint32_t)(slot * 32);
+    constexpr float LOG2E_F = 1.4426950408889634f;
+    for (int i = slot; i < n_items; i += LX_NS) {
+      const long long it = item0 + i;
+      const int b = (int)(it / per_sample), rem = (int)(it % per_sample);
+      const int tile = rem / p.heads, h = rem % p.heads;
+      const int st = i % LX_QS;
+      mbar_wait_sleep(&q_full[st], (uint32_t)((i / LX_QS) & 1), p.wait_ns);
+      // this thread's q row: 8 x 16-byte chunks, chunk c of row r at position c ^ (r & 7) (128-byte swizzle)
+      const uint8_t* qrow = sQ + st * FA_Q_BYTES + r * 128;
+      float x[64];
+#pragma unroll
+      for (int c = 0; c < 8; ++c) unpack8(*reinterpret_cast<const uint4*>(qrow + ((c ^ (r & 7)) << 4)), x + 8 * c);
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&q_empty[st]);
+      // softmax over the head width (dim -1), fp32 with a true max: q is unbounded
+      float m = -INFINITY;
+#pragma unroll
+      for (int d = 0; d < 64; ++d)
+        if (d < p.dim_head) m = fmaxf(m, x[d]);
+      const float mb = m * LOG2E_F;
+      float s = 0.f;
+#pragma unroll
+      for (int d = 0; d < 64; ++d) {
+        x[d] = d < p.dim_head ? ex2_approx(fmaf(x[d], LOG2E_F, -mb)) : 0.f;
+        s += x[d];
+      }
+      const float inv = 1.f / s;
+#pragma unroll
+      for (int half = 0; half < 2; ++half) {
+        uint32_t pk[16];
+#pragma unroll
+        for (int j = 0; j < 16; ++j) pk[j] = pack_bf16x2(x[32 * half + 2 * j] * inv, x[32 * half + 2 * j + 1] * inv);
+        tmem_st16(t_p + (uint32_t)(16 * half), pk);
+      }
+      tmem_st_wait();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&p_full[slot]);
+      mbar_wait_sleep(&o_full[slot], (uint32_t)((i / LX_NS) & 1), p.wait_ns);
+      tc_fence_after();
+      const int row = tile * FA_BM + r;
+      __nv_bfloat16* orow = p.o + (long long)b * p.q_bs + (long long)row * p.q_rs + (long long)h * 64;
+#pragma unroll
+      for (int c0 = 0; c0 < FA_D; c0 += 32) {
+        uint32_t orr[32];
+        tmem_ld32_nowait(t_o + (uint32_t)c0, orr);
+        tmem_ld_wait();
+#pragma unroll
+        for (int j = 0; j < 32; ++j) asm volatile("" : "+r"(orr[j]));
+        if (row < p.rows) {
+#pragma unroll
+          for (int t = 0; t < 4; ++t) {
+            uint4 u;
+            u.x = pack_bf16x2(__uint_as_float(orr[8 * t + 0]), __uint_as_float(orr[8 * t + 1]));
+            u.y = pack_bf16x2(__uint_as_float(orr[8 * t + 2]), __uint_as_float(orr[8 * t + 3]));
+            u.z = pack_bf16x2(__uint_as_float(orr[8 * t + 4]), __uint_as_float(orr[8 * t + 5]));
+            u.w = pack_bf16x2(__uint_as_float(orr[8 * t + 6]), __uint_as_float(orr[8 * t + 7]));
+            *reinterpret_cast<uint4*>(orow + c0 + 8 * t) = u;
+          }
+        }
+      }
+      tc_fence_before();   // the O reads are complete before the next P of this slot lets the issuer overwrite O
+    }
+  }
+  __syncthreads();
+  if (warp == 1) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 512u);
+  }
+}
+
 // 4-D map over [B][rows x heads][64]: dim0 = 64 head channels, dims 1/2 = (rows, heads) ordered by ascending stride
 // (heads_first: the 8 heads of a row are adjacent, as in the cross-attention q / k / v layout), dim3 = batch.
 int encode_rows_map(CUtensorMap* map, const void* base, int rows, int n_heads, int B, long long rs, long long hs, long long bs, int box_rows,
@@ -1403,6 +1656,52 @@ int b200_cross_attention_tc(const void* q, void* o, int64_t q_bs, int64_t q_hs, 
   const int grid = (int)((total + per - 1) / per);
   B200_SMEM_OPT_IN(cross_attn_tc_kernel, XA_SMEM);
   B200_CUDA_OK(b200_launch(cross_attn_tc_kernel, dim3(grid), dim3(64 + 128 * XA_NS), XA_SMEM, st, mq, mk, mv, p));
+  return B200_OK;
+}
+
+extern "C" int b200_linear_xattn_context(const void* k, const void* v, int64_t kv_bs, int32_t kv_rs, int32_t n_keys, int B, int n_heads,
+                                         int32_t dim_head, void* ctx, void* stream) {
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  B200_REQUIRE(k && v && ctx, "linear cross-attention context: null pointer");
+  B200_REQUIRE(n_keys > 0 && B > 0 && B <= 65535 && n_heads > 0 && n_heads <= LX_MAX_HEADS && dim_head > 0 && dim_head <= 64,
+               "linear cross-attention context: bad shape keys=%d B=%d heads=%d dim_head=%d", n_keys, B, n_heads, dim_head);
+  B200_REQUIRE(kv_rs >= n_heads * 64 && kv_bs >= (int64_t)n_keys * kv_rs, "linear cross-attention context: strides too small (rs=%d bs=%lld)",
+               kv_rs, (long long)kv_bs);
+  B200_SMEM_OPT_IN(linear_xattn_context_kernel, LX_CTX_SMEM);
+  B200_CUDA_OK(b200_launch(linear_xattn_context_kernel, dim3(n_heads, B), dim3(LX_CTX_THREADS), LX_CTX_SMEM, st,
+                           reinterpret_cast<const __nv_bfloat16*>(k), reinterpret_cast<const __nv_bfloat16*>(v), (long long)kv_bs, (int)kv_rs,
+                           (int)n_keys, (int)dim_head, reinterpret_cast<__nv_bfloat16*>(ctx)));
+  return B200_OK;
+}
+
+extern "C" int b200_linear_cross_attention(const void* q, void* o, int64_t q_bs, int32_t q_rs, int32_t rows, const void* ctx, int B, int n_heads,
+                                           int32_t dim_head, void* stream) {
+  cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+  B200_REQUIRE(q && o && ctx, "linear cross-attention: null pointer");
+  B200_REQUIRE(rows > 0 && B > 0 && n_heads > 0 && n_heads <= LX_MAX_HEADS && dim_head > 0 && dim_head <= 64,
+               "linear cross-attention: bad shape rows=%d B=%d heads=%d dim_head=%d", rows, B, n_heads, dim_head);
+  B200_REQUIRE((q_rs & 7) == 0 && (q_bs & 7) == 0 && q_rs >= n_heads * 64 && q_bs >= (int64_t)rows * q_rs,
+               "linear cross-attention: strides must be multiples of 8 elements and cover heads x 64 channels (rs=%d bs=%lld)", q_rs, (long long)q_bs);
+  CUtensorMap mq, mc;
+  int rc;
+  if ((rc = encode_rows_map(&mq, q, rows, n_heads, B, q_rs, 64, q_bs, FA_BM, true, "Q")) != B200_OK) return rc;
+  if ((rc = encode_rows_map(&mc, ctx, 64, n_heads, B, 64, 64 * 64, (long long)n_heads * 64 * 64, 64, false, "C")) != B200_OK) return rc;
+  LxParams p;
+  p.o = reinterpret_cast<__nv_bfloat16*>(o);
+  p.q_bs = q_bs; p.q_rs = q_rs; p.rows = rows; p.B = B; p.heads = n_heads; p.dim_head = dim_head;
+  p.tiles_per_sample = (rows + FA_BM - 1) / FA_BM;
+  const long long total = (long long)B * p.tiles_per_sample * n_heads;
+  const int sms = sm_count();
+  long long per = (total + sms - 1) / sms;
+  per = (per + n_heads - 1) / n_heads * n_heads;                 // whole query tiles per CTA: the C reload boundaries fall between tiles
+  p.items_per_cta = (int)per;
+  {
+    static const uint32_t wns = [] { const char* ev = getenv("B200_IMAGEN_FA_WAIT_NS"); return (uint32_t)(ev ? atoi(ev) : FA_DEFAULT_WAIT_NS); }();
+    p.wait_ns = wns;
+  }
+  const int grid = (int)((total + per - 1) / per);
+  B200_SMEM_OPT_IN(linear_cross_attn_tc_kernel, LX_SMEM);
+  B200_CUDA_OK(b200_launch(linear_cross_attn_tc_kernel, dim3(grid), dim3(64 + 128 * LX_NS), LX_SMEM, st, mq, mc, p));
   return B200_OK;
 }
 

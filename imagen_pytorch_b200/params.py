@@ -44,7 +44,7 @@ UNET_DEFAULTS = OrderedDict(
 # Options of the reference constructor that this hot-path implementation does not cover.
 # They raise instead of silently diverging (SURVEY.md section 7 "API edge cases").
 _UNSUPPORTED = dict(
-    use_linear_attn=lambda v: any(cast_tuple(v)), use_linear_cross_attn=lambda v: any(cast_tuple(v)),
+    use_linear_attn=lambda v: any(cast_tuple(v)),
     cross_embed_downsample=bool,
     combine_upsample_fmaps=bool, init_conv_to_final_conv_residual=bool,
     pixel_shuffle_upsample=lambda v: not v, attn_dim_head=lambda v: v > 64 or v < 1,
@@ -105,7 +105,9 @@ class UnetArch:
         self.layer_attns = cast_tuple(g('layer_attns'), n)
         self.layer_attns_depth = cast_tuple(g('layer_attns_depth'), n)
         self.layer_cross_attns = cast_tuple(g('layer_cross_attns'), n)
+        self.use_linear_cross_attn = cast_tuple(g('use_linear_cross_attn'), n)
         assert len(self.layer_attns) == n and len(self.layer_cross_attns) == n and len(self.num_resnet_blocks) == n
+        assert len(self.use_linear_cross_attn) == n
         self.mid_depth = g('layer_mid_attns_depth')
         self.attend_at_middle = bool(g('attend_at_middle'))
         self.init_cross_embed = bool(g('init_cross_embed'))
@@ -121,19 +123,23 @@ class UnetArch:
             raise NotImplementedError('imagen_pytorch_b200.Unet needs dim / init_dim / cond_dim to be multiples of 8 (16-byte NHWC rows)')
 
     # level-wise channel bookkeeping ------------------------------------------------------------
+    def _cross(self, i):
+        """A level has a cross-attention layer when either flag asks for one; use_linear_cross_attn picks LinearCrossAttention
+        (imagen_pytorch.py:1341, :1370, :1395, :1409), which has CrossAttention's parameters."""
+        lin = bool(self.use_linear_cross_attn[i])
+        return dict(cross=bool(self.layer_cross_attns[i]) or lin, linear_cross=lin)
+
     def down_level(self, i):
         dim_in, dim_out = self.in_out[i]
         cur = dim_out if self.memory_efficient else dim_in
-        return dict(dim_in=dim_in, dim_out=dim_out, cur=cur, is_last=i >= self.num_levels - 1,
-                    cross=bool(self.layer_cross_attns[i]), attn=bool(self.layer_attns[i]),
+        return dict(dim_in=dim_in, dim_out=dim_out, cur=cur, is_last=i >= self.num_levels - 1, **self._cross(i), attn=bool(self.layer_attns[i]),
                     depth=self.layer_attns_depth[i], nres=self.num_resnet_blocks[i])
 
     def up_level(self, i):
         lev = self.num_levels - 1 - i
         dim_in, dim_out = self.in_out[lev]
         skip = self.down_level(lev)['cur']
-        return dict(lev=lev, dim_in=dim_in, dim_out=dim_out, skip=skip, is_last=i == self.num_levels - 1,
-                    cross=bool(self.layer_cross_attns[lev]), attn=bool(self.layer_attns[lev]),
+        return dict(lev=lev, dim_in=dim_in, dim_out=dim_out, skip=skip, is_last=i == self.num_levels - 1, **self._cross(lev), attn=bool(self.layer_attns[lev]),
                     depth=self.layer_attns_depth[lev], nres=self.num_resnet_blocks[lev])
 
 

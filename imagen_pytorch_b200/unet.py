@@ -283,8 +283,8 @@ class UnetPlan:
         return out
 
     # ------------------------------------------------------------------ blocks
-    def _resnet(self, p, srcs, dout, *, cross_heads=None, gca=False):
-        """ResnetBlock.forward (imagen_pytorch.py:735-757)."""
+    def _resnet(self, p, srcs, dout, *, cross_heads=None, linear_cross=False, gca=False):
+        """ResnetBlock.forward (imagen_pytorch.py:735-757); linear_cross: LinearCrossAttention instead of CrossAttention (:719)."""
         a, sd, R = self.arch, self.sdc, self.R
         Hc, Wc = srcs[0].H, srcs[0].W
         n = Hc * Wc
@@ -306,7 +306,8 @@ class UnetPlan:
             h = self._new(M, dout, Hc, Wc)
             h.call = self._conv([a1], W1, dout, h.t, ldc=h.ld, bias=b1)
             if cross_heads is not None:
-                a2 = self._cross_attention(p + '.cross_attn', h, cross_heads, g2, film_off)
+                attn = self._linear_cross_attention if linear_cross else self._cross_attention
+                a2 = attn(p + '.cross_attn', h, cross_heads, g2, film_off)
             else:
                 a2 = self._rms_film_silu([h], g2, dout, 1.0, n, film_off)
         W2, b2 = sd[p + '.block2.project.weight'], sd[p + '.block2.project.bias']
@@ -384,24 +385,53 @@ class UnetPlan:
         epilogue of the conv that produced h, and to_out's epilogue does LayerNorm -> + h -> RMSNorm/FiLM/SiLU: 2 launches
         (to_q, attention) + to_out instead of 5 + the block norm."""
         sd, R = self.sdc, self.R
-        n, M, Cc = h.H * h.W, h.rows, h.C
+        n, M = h.H * h.W, h.rows
         inner = heads * 64
         hn = self._prenorm_ln(h, sd[p + '.norm.g'])
-        qs = self._f32(sd[p + '.q_scale'] * (8.0 * LOG2E))
+        qs =self._f32(sd[p + '.q_scale'] * (8.0 * LOG2E))
         q = self._linear(hn, sd[p + '.to_q.weight'], inner, l2_cols=inner, l2_scale=qs)
-        nk = self.n_ctx + 1
-        Kc, Vc = self._zeros((R, nk, inner)), self._zeros((R, nk, inner))
-        Kt, Vt = self._zeros((self.S, self.ntt, inner)), self._zeros((self.S, self.ntt, inner))
-        self.cross_layers.append(dict(p=p, K=Kc, V=Vc, Kt=Kt, Vt=Vt, heads=heads, nk=nk))
-        for tb, dst in ((Kt, Kc), (Vt, Vc)):
-            self._jobs.append(TimeRowJob(tb.data_ptr(), dst.data_ptr(), nk * inner, self.ntt, inner))
-        # static null key/value: last row, same for every head (:805-808)
-        nkv = sd[p + '.null_kv']
-        self._row_fill(Kc[:, nk - 1, :], (F.normalize(nkv[0], dim=-1) * sd[p + '.k_scale']).repeat(heads))
-        self._row_fill(Vc[:, nk - 1, :], nkv[1].repeat(heads))
+        Kc, Vc, nk = self._context_kv(p, heads, linear=False)
         o = self._new(M, inner, h.H, h.W)
         self._add('b200_attention', q.ptr, o.ptr, n * inner, 64, inner, n, Kc.data_ptr(), Vc.data_ptr(), nk * inner, 64, inner, nk, R, heads,
                   self._logit_bound(p))
+        return self._attn_out(p, o, h, g2, film_off)
+
+    def _context_kv(self, p, heads, *, linear):
+        """Per-layer context K/V buffers [R, n_ctx + 1, heads*64]: prepare() writes the static rows, b200_update_time_rows the
+        time-token rows of each sample's schedule slot every step; the null key/value is the last row, the same for every head
+        (:805-808).  CrossAttention stores K l2-normalised * k_scale; LinearCrossAttention (linear=True) uses K raw (:851-866)."""
+        sd, R = self.sdc, self.R
+        inner, nk = heads * 64, self.n_ctx + 1
+        Kc, Vc = self._zeros((R, nk, inner)), self._zeros((R, nk, inner))
+        Kt, Vt = self._zeros((self.S, self.ntt, inner)), self._zeros((self.S, self.ntt, inner))
+        self.cross_layers.append(dict(p=p, K=Kc, V=Vc, Kt=Kt, Vt=Vt, heads=heads, nk=nk, linear=linear))
+        for tb, dst in ((Kt, Kc), (Vt, Vc)):
+            self._jobs.append(TimeRowJob(tb.data_ptr(), dst.data_ptr(), nk * inner, self.ntt, inner))
+        nkv = sd[p + '.null_kv']
+        self._row_fill(Kc[:, nk - 1, :], (nkv[0] if linear else F.normalize(nkv[0], dim=-1) * sd[p + '.k_scale']).repeat(heads))
+        self._row_fill(Vc[:, nk - 1, :], nkv[1].repeat(heads))
+        return Kc, Vc, nk
+
+    def _linear_cross_attention(self, p, h: Rows, heads, g2, film_off):
+        """LinearCrossAttention.forward + residual (imagen_pytorch.py:836-874, :749), followed by block2's norm like _cross_attention:
+        to_q (plain: the softmax over the head width replaces l2norm / q_scale), the per-step context matrix C = 8 softmax_j(k)^T v of
+        every (row, head), O = softmax_d(q) C, and the same to_out epilogue."""
+        sd, R, a = self.sdc, self.R, self.arch
+        n, M = h.H * h.W, h.rows
+        inner = heads * 64
+        hn = self._prenorm_ln(h, sd[p + '.norm.g'])
+        q = self._linear(hn, sd[p + '.to_q.weight'], inner)
+        Kc, Vc, nk = self._context_kv(p, heads, linear=True)
+        ctx = self._zeros((R, heads, 64, 64))
+        self._add('b200_linear_xattn_context', Kc.data_ptr(), Vc.data_ptr(), nk * inner, inner, nk, R, heads, a.dim_head, ctx.data_ptr())
+        o = self._new(M, inner, h.H, h.W)
+        self._add('b200_linear_cross_attention', q.ptr, o.ptr, n * inner, inner, n, ctx.data_ptr(), R, heads, a.dim_head)
+        return self._attn_out(p, o, h, g2, film_off)
+
+    def _attn_out(self, p, o: Rows, h: Rows, g2, film_off):
+        """to_out Linear -> LayerNorm -> + h -> block2's ChanRMSNorm / FiLM / SiLU of a cross-attention layer: returns a2."""
+        sd = self.sdc
+        n, M, Cc = h.H * h.W, h.rows, h.C
         if self._fusable(Cc):
             a2 = self._new(M, Cc, h.H, h.W)
             self._linear(o, sd[p + '.to_out.0.weight'], Cc, out=a2, out_raw=False, norm1=_lib.NORM_LN, norm1_g=self._f32(sd[p + '.to_out.1.g'].flatten()),
@@ -544,7 +574,7 @@ class UnetPlan:
             p = f'downs.{i}'
             if a.memory_efficient:
                 x = self._downsample(p + '.0.1', x, L['dim_out'])
-            x = self._resnet(p + '.1', [x], L['cur'], cross_heads=a.heads if L['cross'] else None)
+            x = self._resnet(p + '.1', [x], L['cur'], cross_heads=a.heads if L['cross'] else None, linear_cross=L['linear_cross'])
             for j in range(L['nres']):
                 x = self._resnet(f'{p}.2.{j}', [x], L['cur'], gca=a.use_gca)
                 hiddens.append(x)
@@ -568,7 +598,8 @@ class UnetPlan:
         for i in range(a.num_levels):                                          # :1698-1708
             U = a.up_level(i)
             p = f'ups.{i}'
-            x = self._resnet(p + '.0', [x, hiddens.pop()], U['dim_out'], cross_heads=a.heads if U['cross'] else None)
+            x = self._resnet(p + '.0', [x, hiddens.pop()], U['dim_out'], cross_heads=a.heads if U['cross'] else None,
+                             linear_cross=U['linear_cross'])
             for j in range(U['nres']):
                 x = self._resnet(f'{p}.1.{j}', [x, hiddens.pop()], U['dim_out'], gca=a.use_gca)
             if U['attn']:
@@ -778,13 +809,14 @@ class UnetPlan:
         for Lr in self.cross_layers:                                            # CrossAttention to_kv of the context (:799-814)
             p, heads, nk = Lr['p'], Lr['heads'], Lr['nk']
             inner = heads * 64
-            Wkv, ksc = sd[p + '.to_kv.weight'], sd[p + '.k_scale']
+            Wkv = sd[p + '.to_kv.weight']
+            knorm, ksc = (False, None) if Lr['linear'] else (True, sd[p + '.k_scale'])   # LinearCrossAttention: raw k (softmax over tokens)
             kvt = self._lin(c_time, Wkv)                                        # [S, ntt, 2*inner]
-            self._store_heads(kvt, 0, heads, True, ksc, Lr['Kt'], 0, ntt, ntt * inner, inner, 64)
+            self._store_heads(kvt, 0, heads, knorm, ksc, Lr['Kt'], 0, ntt, ntt * inner, inner, 64)
             self._store_heads(kvt, inner, heads, False, None, Lr['Vt'], 0, ntt, ntt * inner, inner, 64)
             if ns:
                 kvs = self._lin(ctx_static, Wkv)                                # [R, ns, 2*inner]
-                self._store_heads(kvs, 0, heads, True, ksc, Lr['K'], ntt * inner, ns, nk * inner, inner, 64)
+                self._store_heads(kvs, 0, heads, knorm, ksc, Lr['K'], ntt * inner, ns, nk * inner, inner, 64)
                 self._store_heads(kvs, inner, heads, False, None, Lr['V'], ntt * inner, ns, nk * inner, inner, 64)
         for Ls in self.self_layers:                                             # Attention.to_context (:551-555, :559-561)
             if not Ls['has_ctx']:

@@ -160,6 +160,22 @@ int b200_attention(const void* q, void* o, int64_t q_bs, int64_t q_hs, int32_t q
                    int B, int n_heads, float max_logit, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Linear cross-attention (LinearCrossAttention.forward, imagen_pytorch.py:836-874; Unet(use_linear_cross_attn=...)):
+ *   out = softmax_d(q) @ C,  C[d, e] = 8 * sum_j softmax_j(k)[j, d] * v[j, e]   per (sample b, head h).
+ * Two steps, both per denoising step (the time-token K/V rows change every step):
+ * b200_linear_xattn_context: raw (not normalised) bf16 k / v of problem (b, h) at k + b*kv_bs + h*64, row stride kv_rs,
+ *   n_keys >= 1 rows (the null key/value included) -> ctx, bf16 [B][n_heads][64][64] (row d, column e), rows d >= dim_head zero.
+ * b200_linear_cross_attention: q bf16 rows (problem (b, h) at q + b*q_bs + h*64, row stride q_rs, `rows` pixels), the softmax
+ *   over its first dim_head channels (channels dim_head..63 are zero padding and get weight 0) times ctx -> o, same layout as q.
+ *   tcgen05 kernel: q through a TMA ring, P in tensor memory, O = P C as one M128 x N64 x K64 MMA per 128-row tile.
+ * n_heads <= 8, dim_head <= 64, strides in elements (multiples of 8 for q / o).
+ * ------------------------------------------------------------------------------------------ */
+int b200_linear_xattn_context(const void* k, const void* v, int64_t kv_bs, int32_t kv_rs, int32_t n_keys, int B, int n_heads,
+                              int32_t dim_head, void* ctx, void* stream);
+int b200_linear_cross_attention(const void* q, void* o, int64_t q_bs, int32_t q_rs, int32_t rows, const void* ctx, int B, int n_heads,
+                                int32_t dim_head, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Row-wise normalisation kernels on pixel rows (HBM-bound).
  * ------------------------------------------------------------------------------------------ */
 
